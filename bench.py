@@ -18,6 +18,7 @@ fast mode (one tensor-core pass, ~0.99 label agreement) is timed in the same run
   roofline   : the dominant kernel (tcgen05 implicit-GEMM conv, all launches of a step): algorithmic conv FLOPs /
                summed kernel time, against the measured cuBLAS bf16 peak of MEASURED_PEAKS.json
   cpu_baseline: the oracle (CPU port of the reference math) on a bounded sample, host cores
+  --dump-outputs DIR : after the timed steps, the results of the last step of the `value` region as DIR/<name>.npy
 """
 import argparse
 import json
@@ -94,6 +95,33 @@ def synth_pairs(n, H, W, seed=0):
 def meta(iid, H, W):
     return dict(filename="synthetic_city_%06d.png" % iid, iid=iid, img_shape=(H, W, 3), pad_shape=(H, W, 3),
                 ori_shape=(H, W, 3), scale_factor=1.0)
+
+
+def _sample(t, k, seed):
+    """t itself, or k of its elements at seeded random flat positions when it has more"""
+    if t.numel() <= k:
+        return t
+    idx = torch.randint(t.numel(), (k,), generator=torch.Generator().manual_seed(seed))
+    return t.reshape(-1)[idx.to(t.device)]
+
+
+def result_arrays(r):
+    """the arrays a caller of the timed path receives for one pair (bbox_results, segm_results, pano_results), as
+    float32 / float64 numpy arrays, at most ~34 MB in all: label maps up to 4M pixels whole (a seeded sample beyond),
+    a seeded 64K-element sample of each FPN level.  Copied at once: the runner reuses its output buffers."""
+    bbox, _, pano = r
+    ids = sorted(bbox)
+    out = {"bbox_ids": np.array(ids, np.float64),
+           "bbox_labels": np.array([bbox[i]["label"] for i in ids], np.float64),
+           "bbox": np.array([bbox[i]["bbox"] for i in ids], np.float32).reshape(-1, 4)}
+    for name in ("panoptic_outputs", "fcn_outputs"):
+        out[name] = _sample(pano[name], 1 << 22, 0).cpu().numpy().astype(np.float32)
+    for name in ("panoptic_cls_inds", "panoptic_det_labels", "panoptic_det_obj_ids"):
+        out[name] = pano[name].cpu().numpy().astype(np.float64)
+    out["panoptic_cls_prob"] = pano["panoptic_cls_prob"].cpu().numpy().astype(np.float32)
+    for lvl, f in enumerate(pano["fpn_feats"]):
+        out["fpn_feats_%d_sample" % lvl] = _sample(f.float(), 1 << 16, 1 + lvl).cpu().numpy()
+    return out
 
 
 # ------------------------------------------------------------------------------------------------ CPU arms
@@ -275,6 +303,7 @@ def run_gpu_arm(args):
     # viper: streaming clips -- the reference frame of frame t is frame t - 1 (cityscapes_vps.py:137-142), so the runner
     # reuses the previous pair's FPN features as reference features (results bit-identical: tests/test_gpu_e2e.py)
     runner = ClipRunner(det, dev, streaming=viper)
+    last = {}                                        # the most recent result a region yielded
 
     def region(n, offset, resident):
         src = devp if resident else host
@@ -293,6 +322,7 @@ def run_gpu_arm(args):
         chk = 0
         for r in runner.run(pairs, metas, resident=resident):
             chk += int(r[2]["panoptic_outputs"][0, 0, 0])       # the maps are host tensors here
+            last["r"] = r
         e.record()
         torch.cuda.synchronize()
         return s.elapsed_time(e)
@@ -309,6 +339,7 @@ def run_gpu_arm(args):
     l0 = ops.launch_count()
     ms = [region(args.steps, args.warmup + 5, True)]
     launches = ops.launch_count() - l0
+    dump = result_arrays(last["r"]) if args.dump_outputs and rank == 0 else None
     torch.cuda.synchronize()
     P.barrier()
     ms_e2e = [region(args.steps, args.warmup + 5 + args.steps, False)]
@@ -509,6 +540,10 @@ def run_gpu_arm(args):
             except Exception as ex:          # context only: never fail the bench on it
                 line["stock_pytorch_r50fpn"] = {"unavailable": repr(ex)[:200]}
         print(json.dumps(line))
+    if dump is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dump.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     P.barrier()
     if world > 1:
         import torch.distributed as dist
@@ -531,6 +566,10 @@ def main():
                     help="pairs = BASELINE config 2 (1024x2048 pairs); viper = config 4 (30-frame 1088x1920 clips, one per GPU)")
     ap.add_argument("--allow-short-warmup", action="store_true", help="profiling runs under ncu only (numbers are not bench values)")
     ap.add_argument("--profile-out", default="", help="write per-call device timings of one instrumented step (JSON lines)")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write the results of the last step of the headline timed region (rank 0) as DIR/<name>.npy "
+                         "(float32 / float64; label maps whole, seeded samples of the FPN features): the inputs are "
+                         "seeded, so two builds run with the same arguments can be compared output for output")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if (args.impl == "b200" and not args.allow_short_warmup) else args.warmup
     if args.impl == "reference":

@@ -14,10 +14,12 @@ from vps_b200.synth import init_weights  # noqa: F401  (shared, model-agnostic p
 
 
 @torch.no_grad()
-def calibrate(model, size=(128, 256), seed=123):
+def calibrate(model, size=(128, 256), seed=123, scales=None):
     """Data-dependent rescaling (LSUV-style) so the synthetic network is numerically non-degenerate:
     O(1) pyramid features, sub-pixel..pixel flows, un-saturated class scores, O(1) mask logits and
-    tracker scores.  Deterministic (fixed seed, CPU fp32).  Only linear output layers are rescaled."""
+    tracker scores.  Deterministic (fixed seed, CPU fp32).  Only linear output layers are rescaled.
+    Returns the factors applied, in order.  The measured factors differ in their last bits between hosts (thread count,
+    CPU kernels); `scales`, such a list from an earlier run, is applied instead of them: that run's weights, bit for bit."""
     import torch.nn.functional as F
     from . import model as M
     g = torch.Generator().manual_seed(seed)
@@ -25,7 +27,12 @@ def calibrate(model, size=(128, 256), seed=123):
     img = torch.randn(1, 3, H, W, generator=g)
     ref = torch.roll(img, shifts=(1, 2), dims=(2, 3)) + 0.05 * torch.randn(1, 3, H, W, generator=g)
 
+    applied = []
+
     def scale_(mod, s):
+        if scales is not None:
+            s = float(scales[len(applied)])
+        applied.append(s)
         mod.weight.mul_(s)
         if getattr(mod, "bias", None) is not None:
             mod.bias.mul_(s)
@@ -90,14 +97,20 @@ def calibrate(model, size=(128, 256), seed=123):
     mf = M.roi_extract(xf[:4], rois[:32], 14)
     ms = model.mask_head(mf)
     scale_(model.mask_head.conv_logits, 2.0 / max(ms.pow(2).mean().sqrt().item(), 1e-6))
-    return model
+    assert scales is None or len(scales) == len(applied)
+    return applied
 
 
-def make_model(kind="C", seed=0, calibrated=True, cache_dir="/tmp/vps_oracle_weights"):
-    """Oracle model with synthetic weights; the calibrated state_dict is cached on disk."""
+def make_model(kind="C", seed=0, calibrated=True, cache_dir="/tmp/vps_oracle_weights", scales=None):
+    """Oracle model with synthetic weights; the calibrated state_dict is cached on disk.  `scales`: calibrate() replays
+    these factors (no cache)."""
     import os
     from .model import PanopticFuseTrack
     m = PanopticFuseTrack()
+    if scales is not None:
+        init_weights(m, kind, seed)
+        calibrate(m, scales=scales)
+        return m
     path = os.path.join(cache_dir, "w_%s_%d_%d.pt" % (kind, seed, int(calibrated)))
     if os.path.exists(path):
         m.load_state_dict(torch.load(path))

@@ -17,12 +17,25 @@ import torch
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, ROOT)
 
-from oracle.weights import make_model  # noqa: E402
+from oracle.weights import calibrate, make_model  # noqa: E402
 from tests.e2e_util import make_pair, meta  # noqa: E402
 from tests.golden.run_reference import build_reference_detector  # noqa: E402
 
 H, W = 128, 256
 OUT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "fusetrack_clip_128x256.npz")
+# host threads of the golden run: the summation order of the CPU kernels, hence the last bits of every float, depends on
+# it; tests/test_golden_cpu.py runs the oracle with as many
+THREADS = 8
+
+
+def keep(name, a):
+    """the part of an intermediate tensor ([N, C, H, W] maps, [rows, C] cls_score) the golden file stores, which keeps the
+    file small: every 4th pixel each way of the maps (and every 16th channel of fused0), every 2nd row of cls_score"""
+    if name == "cls_score":
+        return a[::2]
+    if name == "fused0":
+        a = a[:, ::16]
+    return a[..., ::4, ::4]
 
 
 def weights_digest(sd):
@@ -34,7 +47,9 @@ def weights_digest(sd):
 
 
 def main():
-    oracle = make_model("C", 0)
+    torch.set_num_threads(THREADS)
+    oracle = make_model("C", 0, calibrated=False)
+    scales = calibrate(oracle)
     sd = oracle.state_dict()
     det = build_reference_detector(sd)
     cap = {}
@@ -46,7 +61,7 @@ def main():
     det.bbox_head.register_forward_hook(_first_cls)
     det.extra_neck.register_forward_hook(lambda m, i, o: cap.__setitem__("fused0", o[0].detach().clone()))
     img, ref = make_pair(H, W)
-    out = {"weights_sha256": np.array(weights_digest(sd)), "H": H, "W": W}
+    out = {"weights_sha256": np.array(weights_digest(sd)), "calib_scales": np.array(scales, np.float64), "H": H, "W": W}
     with torch.no_grad():
         for f, (iid, a, b) in enumerate(((10001, img, ref), (10002, ref, img))):
             cap.clear()
@@ -61,10 +76,8 @@ def main():
             ids = sorted(r[0].keys())
             out["f%d_bbox_ids" % f] = np.array(ids, np.int32)
             out["f%d_bbox" % f] = np.stack([r[0][i]["bbox"] for i in ids]).astype(np.float32)
-            out["f%d_flow_full" % f] = cap["flow_full"].numpy().astype(np.float32)
-            out["f%d_fcn_score" % f] = cap["fcn_score"].numpy().astype(np.float32)
-            out["f%d_cls_score" % f] = cap["cls_score"].numpy().astype(np.float32)
-            out["f%d_fused0" % f] = cap["fused0"][:, ::16].numpy().astype(np.float32)   # every 16th channel
+            for name in ("flow_full", "fcn_score", "cls_score", "fused0"):
+                out["f%d_%s" % (f, name)] = keep(name, cap[name].numpy()).astype(np.float32)
     np.savez_compressed(OUT, **out)
     print("wrote", OUT, os.path.getsize(OUT) // 1024, "KiB")
 

@@ -11,6 +11,7 @@ import pytest
 import torch
 
 from tests.e2e_util import build_models, compare_frame, make_pair, meta
+from tests.golden.make_golden import keep
 
 pytestmark = pytest.mark.gpu
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "fusetrack_clip_128x256.npz")
@@ -65,9 +66,9 @@ def test_fp32_clip_matches_reference_golden(models, precision):
         ids = sorted(r[0].keys())
         assert ids == g["f%d_bbox_ids" % f].tolist()
         assert np.abs(np.stack([r[0][i]["bbox"] for i in ids]) - g["f%d_bbox" % f]).max() <= 5e-3
-        fs = taps["fcn_score"].float().permute(0, 3, 1, 2).cpu().numpy()
+        fs = keep("fcn_score", taps["fcn_score"].float().permute(0, 3, 1, 2).cpu().numpy())
         assert np.abs(fs - g["f%d_fcn_score" % f]).max() <= 1e-3
-        fl = taps["flow_full"].permute(0, 3, 1, 2).cpu().numpy()
+        fl = keep("flow_full", taps["flow_full"].permute(0, 3, 1, 2).cpu().numpy())
         assert np.abs(fl - g["f%d_flow_full" % f]).max() <= 1e-3
 
 
