@@ -102,13 +102,15 @@ int64_t vps_packed_tc_bytes(int cout, int cin, int kh, int kw, int cin_gran);
 /* ---- fp32-parity tensor-core convolution ("tc32" precision) ------------------------------------
  * Same contract as vps_conv2d_tc, but x (and y, res) are fp32: the reference's convolutions are fp32 cuDNN calls
  * (resnet.py:506-517, flownet2.py:133-198, fpn.py:100-139 ...) and north_star asks for label maps / ids bit-exact.
- * Each operand is split on the fly into fp16(v) + bf16 corrections and three tcgen05 products
- *   fp16(a)*fp16(b) + bf16(a - fp16(a))*bf16(b) + bf16(a)*bf16(b - fp16(b))
- * are summed (~2^-21 relative per product, 3 tensor-core passes).  Because tcgen05.mma truncates when it adds into its
- * accumulator, the main product is accumulated in short chains that are promoted to round-to-nearest register sums
- * (conv_tc32.cu).  Weights are pre-split by vps_pack_weights_tc32 into [fp16 | bf16 | bf16] planes; the nprob stride
- * phases of a transposed convolution share ONE packed buffer (args[i].w identical, problem i = plane slice i).
- * |value| > 65504 in x or w saturates the fp16 plane (the result then carries ~8 correct bits) and is counted:
+ * Each operand is split on the fly into two fp16 planes, v = A + 2^-11 * A2 with A = fp16(v), A2 = fp16(2^11 (v - A)),
+ * and three tcgen05 products
+ *   A*B + 2^-11 * (A2*B + A*B2)
+ * are summed (~2^-21 relative per product, 3 tensor-core passes; below 2^-14 an operand carries an absolute error of
+ * 2^-36).  Because tcgen05.mma truncates when it adds into its accumulator, the main product is accumulated in short chains
+ * that are promoted to round-to-nearest register sums (conv_tc32.cu).  Weights are pre-split by vps_pack_weights_tc32 into
+ * two fp16 planes [B | B2]; the nprob stride phases of a transposed convolution share ONE packed buffer (args[i].w
+ * identical, problem i = plane slice i).
+ * |value| > 65504 (or NaN) in x or w saturates the fp16 planes (the result is then wrong) and is counted:
  * vps_tc32_overflow(reset) returns the count (device sync) -- callers must treat non-zero as an error. */
 int vps_conv2d_tc32(const vps_conv_args* a, void* stream);
 int vps_conv2d_tc32_multi(const vps_conv_args* a, int nprob, void* stream);

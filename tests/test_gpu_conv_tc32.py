@@ -1,6 +1,8 @@
-"""GPU parity of the fp32-parity tensor-core convolution (vps_conv2d_tc32: tf32 + two bf16 correction products per
-K slab) vs fp64 convolution on the CPU.  Tolerance: 2e-5 of the output scale -- fp32-class (the CUDA-core fp32 kernel is
-held to 1e-4 in test_gpu_conv.py), 100x below what one bf16 pass gives (2e-3)."""
+"""GPU parity of the fp32-parity tensor-core convolution (vps_conv2d_tc32: every operand split into two fp16 planes,
+v = fp16(v) + 2^-11 fp16(2^11 (v - fp16(v))), three products per K slab) vs fp64 convolution on the CPU, over the layer
+shapes of the model.  Tolerance: 2e-5 of the output scale -- fp32-class (the CUDA-core fp32 kernel is held to 1e-4 in
+test_gpu_conv.py), 100x below what one bf16 pass gives (2e-3).  The elementwise error bound, the truncation bias, the
+fp16 range edges, the saturation counter and the rarer epilogue paths are tested in test_gpu_tc32_numerics.py."""
 import pytest
 import torch
 import torch.nn.functional as F

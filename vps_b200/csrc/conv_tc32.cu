@@ -235,7 +235,7 @@ __device__ __forceinline__ void producer32(const ConvTcParams& p, const Tc32Extr
   }
 }
 
-// ---------------------------------------------------------------- warps 2..7: fp32 box -> fp16 / bf16 / bf16 operand planes
+// ---------------------------------------------------------------- warps 3..7: fp32 box -> the two fp16 operand planes
 __device__ __forceinline__ void converter32(const ConvTcParams& p, const Tc32Extra& e, const Ring32& rg, int ctid, int nthreads) {
   const int ntaps = p.kh * p.kw;
   const int items_per_tile = p.cin_chunks * (p.halo ? 1 : ntaps);
@@ -627,6 +627,16 @@ __device__ __forceinline__ void epi_chunk_tma(const ConvTcParams& p, const CUten
   asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
   __syncwarp();
   if (lane == 0) tma_store_4d(tmY, scratch, n0, x0, y0, img);
+  // the TMA clips the channel axis in 16-byte units, so its tensor map ends at cout & ~3: the last cout % 4 channels are
+  // stored per lane
+  const int tail = p.cout & 3;
+  if (!PLAIN && tail && nlim == p.cout && valid) {
+    const int j0 = (nlim & ~3) - n0;
+    float* yp = (float*)p.y + pix * p.y_cs + n0;
+#pragma unroll
+    for (int j = 0; j < 32; ++j)
+      if (j >= j0 && j < j0 + tail) yp[j] = v[j];
+  }
 }
 
 // ---------------------------------------------------------------- warps 8..15: promotion (TMEM groups -> register sums) + epilogue
@@ -1097,20 +1107,25 @@ extern "C" int vps_conv2d_tc32_multi(const vps_conv_args* args, int nprob, void*
     if (epi_env < 0) { const char* ev = getenv("VPS_TC32_EPI"); epi_env = ev ? atoi(ev) : 2; }
     const bool y_ok = a->y.dtype == VPS_F32 && (((uintptr_t)a->y.ptr & 15) == 0) && (a->y.cs % 4 == 0);
     const bool r_ok = !a->res.ptr || (a->res.dtype == VPS_F32 && (((uintptr_t)a->res.ptr & 15) == 0) && (a->res.cs % 4 == 0));
-    p.epi_t = (y_ok && r_ok && a->y.c == a->cout && epi_env >= 2) ? 2 : 0;
+    // the TMA clips a box at the end of the channel axis only in 16-byte units (a map ending at cout % 4 != 0 wrote up to 3
+    // channels past cout, into neighbouring slices of a concat buffer): the map ends at cout & ~3, epi_chunk_tma stores the rest
+    p.epi_t = (y_ok && r_ok && a->y.c == a->cout && a->cout >= 4 && epi_env >= 2) ? 2 : 0;
   }
-  const int smem_budget = 227 * 1024 - 1024 - T32_BAR_BYTES - 64 - (p.epi_t == 2 ? (int)T32_SCRATCH_BYTES : 0);
   const int a_side = T32_STAGE_SLOTS * e.stage_bytes + p.a_stages * p.a_stage_bytes;
   // N tile: divisor of cout_pad (multiple of 16, <= 128) minimising waves * (steps * step clocks + epilogue); a step is
-  // 6 MMAs = 3*bn clocks at the MMA floor, ~300 clocks of issue / barrier latency, or its weight bytes at the L2 rate
-  int block_n = 16;
-  {
+  // 6 MMAs = 3*bn clocks at the MMA floor, ~300 clocks of issue / barrier latency, or its weight bytes at the L2 rate.
+  // The TMA-store epilogue writes 32-channel boxes that are clipped only at the END of the tensor's channel axis, so it needs
+  // bn % 32 == 0 or a single N tile; when cout_pad > 128 has no such divisor (cout_pad / 16 odd: cout 144, 176, 208, ...)
+  // every N tile but the last would write 16 stale channels over its neighbour's, and the scalar epilogue is used instead.
+  int block_n = 0, smem_budget = 0;
+  for (int pass = 0; pass < 2 && block_n == 0; ++pass) {
+    if (pass == 1) p.epi_t = 0;
+    smem_budget = 227 * 1024 - 1024 - T32_BAR_BYTES - 64 - (p.epi_t == 2 ? (int)T32_SCRATCH_BYTES : 0);
     const int64_t m_tiles = (int64_t)a->x.n * p.tiles_y * p.tiles_x * nprob;
     double best = -1.0;
     for (int bn = 16; bn <= T32_MAX_N && bn <= cout_pad; bn += 16) {
       if (cout_pad % bn) continue;
       if (a_side + 2 * bn * 64 * T32_PLANES > smem_budget) continue;
-      // TMA-store epilogue: boxes are 32 channels wide and only clipped at the END of the tensor's channel axis
       if (p.epi_t == 2 && (bn % 32) && bn != cout_pad) continue;
       const int64_t tiles = m_tiles * (cout_pad / bn);
       const double waves = (double)((tiles + g_num_sms32 - 1) / g_num_sms32);
@@ -1119,6 +1134,7 @@ extern "C" int vps_conv2d_tc32_multi(const vps_conv_args* args, int nprob, void*
       if (best < 0 || t < best * 0.999) { best = t; block_n = bn; }
     }
   }
+  VPS_CHECK_ARG(block_n > 0, "conv2d_tc32: no N tile fits (%d x %d px halo, cout %d)", halo_h, p.halo_w, a->cout);
   p.block_n = block_n; p.n_tiles_n = cout_pad / block_n;
   e.b_plane_bytes = block_n * 64;
   {
@@ -1202,7 +1218,7 @@ extern "C" int vps_conv2d_tc32_multi(const vps_conv_args* args, int nprob, void*
     const int bw = p.tw < 32 ? p.tw : 32, bh = 32 / bw;
     for (int i = 0; i < nprob; ++i) {
       const vps_conv_args* q = &args[i];
-      cuuint64_t dims[4] = {(cuuint64_t)a->cout, (cuuint64_t)a->ow, (cuuint64_t)a->oh, (cuuint64_t)a->y.n};
+      cuuint64_t dims[4] = {(cuuint64_t)(a->cout & ~3), (cuuint64_t)a->ow, (cuuint64_t)a->oh, (cuuint64_t)a->y.n};
       cuuint64_t strides[3] = {(cuuint64_t)a->ox_mul * a->y.cs * 4, (cuuint64_t)a->oy_mul * a->y.w * a->y.cs * 4,
                                (cuuint64_t)a->y.h * a->y.w * a->y.cs * 4};
       cuuint32_t box[4] = {32, (cuuint32_t)bw, (cuuint32_t)bh, 1};
@@ -1341,6 +1357,7 @@ extern "C" int vps_deform_conv_tc32(const vps_tensor* x, const vps_tensor* offse
     (void)epi_env;
     VPS_CHECK_ARG(y->dtype == VPS_F32 && (((uintptr_t)y->ptr & 15) == 0) && (y->cs % 4 == 0),
                   "deform_conv_tc32: y must be fp32 with 16-byte aligned pixel rows (cs=%d)", y->cs);
+    VPS_CHECK_ARG(cout % 4 == 0, "deform_conv_tc32: cout %d: the TMA epilogue clips channels in 16-byte units", cout);
     p.epi_t = 2;
   }
   static int dcn_a_env = -1, dcn_b_env = -1;

@@ -1,5 +1,5 @@
 // Shared device code of the tcgen05 implicit-GEMM kernels (conv_tc.cu: bf16 operands; conv_tc32.cu: fp32 operands
-// split on the fly into tf32 + bf16 correction planes): launch parameters, PTX wrappers (mbarrier / TMA / tcgen05),
+// split on the fly into two fp16 planes, v = fp16(v) + 2^-11 fp16(2^11 (v - fp16(v)))): launch parameters, PTX wrappers (mbarrier / TMA / tcgen05),
 // and the epilogue (TMEM -> bias / activation / residual -> NHWC store).
 #pragma once
 #include <cudaTypedefs.h>

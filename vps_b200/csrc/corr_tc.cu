@@ -383,7 +383,8 @@ extern "C" int64_t vps_correlation_tc32_ws_bytes(const vps_tensor* f1) {
 // (v = hi + 2^-11 lo) and the banded GEMM runs three times, hi.hi, then hi.lo and lo.hi scaled by 2^-11 and accumulated
 // into the fp32 output (the activation is applied by the last pass).  Unlike the stacked convolutions a correlation is a
 // single K = C <= 256 contraction (16 MMAs per accumulator chain) whose result is not fed through further layers of the same
-// kind, so the tensor core's truncating accumulation (~3e-7 relative over such a chain) needs no promotion here.
+// kind, so the tensor core's truncating accumulation needs no promotion here (measured on a B200 at C = 256 with
+// all-positive features: mean relative error -1.2e-6, max 1.4e-6 of sum |f1 f2| / C; the promoted convolutions: -7e-8).
 // `ws`: vps_correlation_tc32_ws_bytes() of scratch, 256-byte aligned.  Same supported geometries as vps_correlation_tc.
 extern "C" int vps_correlation_tc32(const vps_tensor* f1, const vps_tensor* f2, const vps_tensor* out, int pad, int max_disp,
                                     int stride1, int stride2, int act, float slope, void* ws, void* stream) {

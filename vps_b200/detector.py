@@ -10,8 +10,8 @@ names, so `state_dict()` keys match a reference checkpoint.  Differences by desi
     (NMS mask download, MaskROI numpy, MaskRemoval numpy/cv2, SegTerm numpy, tracker loops) are kernels.
     Two 4-byte counters (number of detections, tracker memory size) are read back per frame to size the
     data-dependent launches.
-  * `precision`: "tc32" (fp32 activations, tcgen05 tensor cores with split operands: tf32 + two bf16 correction
-    products per K slab -- the parity mode, label maps / ids bit-exact vs the oracle), "bf16" (bf16 activations, one
+  * `precision`: "tc32" (fp32 activations, tcgen05 tensor cores with split operands: two fp16 planes per
+    operand, v = fp16(v) + 2^-11 fp16(2^11 (v - fp16(v))), three products per K slab -- the parity mode, label maps / ids bit-exact vs the oracle), "bf16" (bf16 activations, one
     tensor-core pass: fastest, ~1e-2 relative on features) or "fp32" (CUDA-core fp32 FMA: debugging reference).
 """
 import numpy as np
@@ -348,6 +348,11 @@ class PanopticFuseTrack(nn.Module):
         ops.SCOPE[0] = 'track_mask_fuse'
         k, dummy = [int(v) for v in kout.tolist()]            # 8-byte read-back: number of detections
         if self.precision == "tc32" and ops.tc32_overflow():
+            # leave the detector usable (e.g. for the fp32 rerun suggested below): drop the static parts prefetch() enqueued
+            # for later frames, and clear the counts their kernels may still add once they finish
+            self._pf_queue.clear()
+            torch.cuda.synchronize(dev)
+            ops.tc32_overflow(reset=True)
             raise ops.VpsError("tc32: an activation or weight exceeded the fp16 range (65504) of the main tensor-core "
                                "product; use precision='fp32' for this input")
         iid = meta['iid']

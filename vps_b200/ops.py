@@ -157,7 +157,8 @@ class PackedConv:
         return self._tc[gran]
 
     def tc32(self):
-        """[fp16 | bf16 | bf16] planes of the fp32-parity tensor-core kernel (vps_conv2d_tc32)."""
+        """[B | B2] fp16 planes of the fp32-parity tensor-core kernel (vps_conv2d_tc32): B = fp16(w * scale),
+        B2 = fp16(2^11 (w * scale - B)), the scale folded in fp32."""
         if self._tc32 is None:
             self._tc32 = pack_tc32([self])
         return self._tc32
